@@ -2,6 +2,7 @@
 """bench.py — SeedVR2-3B upscaled frames/s on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N --steps K --warmup W] [--workload 4k_shard|1080p|...] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (VAE encode -> DiT one-step -> VAE decode)
 over one clip of synthetic video per GPU.  Default workload = the per-GPU shard
@@ -16,6 +17,9 @@ the decoded frames.  Output: ONE JSON line on rank 0 (see the task contract).
   roofline : the tcgen05 GEMM/implicit-conv kernel (dominant): algorithmic FLOPs of
           all its launches / their CUDA-event time, vs the measured bf16 peak
   cpu_baseline : the oracle port (torch fp32, all host threads) on a bounded sample
+
+--dump-outputs DIR writes what the last timed step of `value` returned (rank 0) as DIR/<name>.npy in float32, so that
+two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -26,6 +30,9 @@ import subprocess
 import sys
 import threading
 import time
+
+# the tree the benchmark runs from may be read-only: no bytecode caches written next to the sources
+sys.dont_write_bytecode = True
 
 # Clips that fill the HBM (temporally sliced VAE passes sized from the free memory) need an allocator that does not
 # fragment: expandable segments, chosen before torch initialises CUDA.  The default workloads keep torch's default.
@@ -65,6 +72,22 @@ def flop_model(frames_pad: int, H: int, W: int, variant="3b"):
     attn_vae = T_lat * (4.0 * n * n * 512 + 8.0 * n * 512 * 512)
     return dict(dit=per_tok * L, enc=9.0e6 * frames_pad * Hp * Wp + attn_vae,
                 dec=24.2e6 * frames_pad * Hp * Wp + attn_vae, tokens=L)
+
+
+DUMP_SAMPLE = 8 * 2**20         # elements kept of an output larger than that: 32 MiB of float32 per array
+
+
+def dump_outputs(path, arrays):
+    """Each tensor as path/<name>.npy in float32: whole when it has at most DUMP_SAMPLE elements, else the elements at
+    DUMP_SAMPLE sorted flat indices drawn from a fixed seed (the same positions for every build of one workload)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def synth_frames(T, H, W, seed=42, device="cpu"):
@@ -223,7 +246,12 @@ def main():
                          "metric is quoted with 'none' = the north_star path (encode + DiT + decode)")
     ap.add_argument("--phases", action="store_true", help="print a per-kernel breakdown to stderr")
     ap.add_argument("--detail", action="store_true", help="with --phases: break GEMM/conv launches down by shape")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32; a fixed, seeded sample "
+                         f"of {DUMP_SAMPLE} elements of a larger output)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     frames_real, H, W, desc = WORKLOADS[args.workload]
     vae_only = args.workload.startswith("vae_decode")
     from svr2_import import load_package
@@ -290,13 +318,18 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(args.steps):
-        step(frames_dev)
+    for i in range(args.steps):
+        y = step(frames_dev)
+        if i + 1 < args.steps:          # only the last step's result stays alive
+            del y
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = lib.LAUNCHES
     peak_mem_native = torch.cuda.max_memory_allocated()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"sample" if vae_only else "frames": y})
+    del y
     # ---- region P: the same steps with per-kernel CUDA events on the launching stream (per-call events need the Python
     # sequencing of the same kernels): the roofline and the per-kernel table come from here, not the headline value
     prof_steps = 1 if ms / args.steps > 5000 else min(args.steps, 3)      # long clips: one profiled pass is enough

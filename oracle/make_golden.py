@@ -23,7 +23,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from oracle import dit_oracle, vae_oracle  # noqa: E402
+from oracle import dit_oracle, dropin, vae_oracle  # noqa: E402
 from oracle import ref_import  # noqa: E402
 from oracle.ref_import import import_reference_dit, import_reference_vae  # noqa: E402
 from svr2_import import load_package  # noqa: E402
@@ -334,11 +334,14 @@ def main():
     torch.manual_seed(0)
     if "--tiled-only" in sys.argv:
         return run_tiled_cases()
+    if "--dropin-only" in sys.argv:
+        return dropin.record_reference(pkg, os.path.join(GOLD, "dropin_runner.npz"))
     if "--color-only" not in sys.argv and "--pre-only" not in sys.argv:
         for name in DIT_CASES:
             run_dit_case(name)
         run_vae_cases()
         run_tiled_cases()
+        dropin.record_reference(pkg, os.path.join(GOLD, "dropin_runner.npz"))
     if "--pre-only" not in sys.argv:
         run_color_cases()
     if "--color-only" not in sys.argv:

@@ -1,157 +1,87 @@
-"""CPU (build container only): the engine's model-slot modules dropped into the REFERENCE's own pipeline objects.
+"""CPU: the engine's model-slot modules against a record of the REFERENCE's own pipeline objects driving them.
 
-The reference's ``VideoDiffusionInfer`` (``src/core/infer.py``) and its memory manager (``src/optimization/memory_manager.py``)
-are imported from ``/root/reference`` through the test-only stubs of ``oracle/ref_import.py`` (+ a dict-backed
-``omegaconf`` shim); ``runner.dit`` / ``runner.vae`` are the engine's ``B200NaDiT`` / ``B200VideoVAE``.  There is no GPU
-here, so the engine's kernel calls are monkeypatched: the forwards delegate to the (reference-pinned) oracle on the same
-weights.  What is under test is everything BETWEEN the reference and the kernels: the call contract of the slots
-(``infer.py:117-199, 203-278, 315-395``: argument names, shapes, dtypes, the ``tiled`` / ``tile_size`` / ``tile_overlap``
-keywords, ``.latent`` / ``.sample`` / ``.vid_sample``), the ``nn.Module`` surface the pipeline relies on
-(``parameters()`` sniffing, ``named_modules()``, ``.to()``, ``requires_grad_().eval()``) and the lifecycle
-(``manage_model_device``, ``clear_rope_lru_caches``, ``cleanup_dit`` / ``release_model_memory``,
-``memory_manager.py:427-455, 544-581, 670-738, 1011-1097``).  ``/root/reference`` does not exist on the GPU box: skipped there.
+``tests/golden/dropin_runner.npz`` was recorded (``python -m oracle.make_golden --dropin-only``, ``oracle/dropin.py``) by
+running the reference's ``VideoDiffusionInfer`` (``src/core/infer.py``) with ``runner.dit`` / ``runner.vae`` set to the
+engine's ``B200NaDiT`` / ``B200VideoVAE`` on one seeded clip, and its memory manager's lifecycle functions
+(``src/optimization/memory_manager.py``) on those modules.  There is no GPU here, so the engine's kernel calls are replaced
+by the (reference-pinned) oracle on the same weights.  What is under test is everything BETWEEN the reference and the
+kernels: the call contract of the slots (``infer.py:117-199, 203-278, 315-395``: argument names, shapes, dtypes, the
+``tiled`` / ``tile_size`` / ``tile_overlap`` keywords, ``.latent`` / ``.sample`` / ``.vid_sample``), the engine's own clip
+runner (``pipeline.SeedVR2Engine``, which mirrors ``VideoDiffusionInfer``) against the reference runner's results, the
+``nn.Module`` surface the pipeline relies on (``parameters()`` sniffing, ``named_modules()``, ``.to()``,
+``requires_grad_().eval()``) and the lifecycle (``manage_model_device``, ``clear_rope_lru_caches``, ``cleanup_dit`` /
+``release_model_memory``, ``memory_manager.py:427-455, 544-581, 670-738, 1011-1097``) as the module calls they make.
 """
 import importlib
+import inspect
+import json
 import os
-import sys
-import types
 
+import numpy as np
 import pytest
 import torch
-import yaml
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="reference tree not present")
+from oracle import dropin
 
-
-class Cfg(dict):
-    """dict-backed stand-in for omegaconf.DictConfig: attribute access, .get, nested."""
-
-    def __init__(self, d=None):
-        super().__init__()
-        for k, v in (d or {}).items():
-            self[k] = Cfg(v) if isinstance(v, dict) else v
-
-    def __getattr__(self, k):
-        try:
-            return self[k]
-        except KeyError as e:
-            raise AttributeError(k) from e
-
-    def __setattr__(self, k, v):
-        self[k] = v
-
-
-class ListCfg(list):
-    pass
-
-
-class Debug:
-    def log(self, *a, **k):
-        pass
-
-    def start_timer(self, *a, **k):
-        pass
-
-    def end_timer(self, *a, **k):
-        return 0.0
-
-    def log_memory_state(self, *a, **k):
-        pass
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dropin_runner.npz")
 
 
 @pytest.fixture(scope="module")
-def ref():
-    from oracle import ref_import
-    ref_import.install_stubs()
-    om = types.ModuleType("omegaconf")
-    om.DictConfig, om.ListConfig = Cfg, ListCfg
-    om.OmegaConf = types.SimpleNamespace(load=lambda p: Cfg(yaml.safe_load(open(p))), create=lambda x: Cfg(x),
-                                         register_new_resolver=lambda *a, **k: None)
-    sys.modules.setdefault("omegaconf", om)
-    infer = importlib.import_module("src.core.infer")
-    mm = importlib.import_module("src.optimization.memory_manager")
-    cfg = Cfg(yaml.safe_load(open(os.path.join(REF, "configs_3b", "main.yaml"))))
-    cfg.vae.dtype = "bfloat16"
-    cfg.diffusion.cfg.scale = 1.0                      # generation_phases.py:598-601: one-step, cfg 1
-    cfg.diffusion.timesteps.sampling.steps = 1
-    return types.SimpleNamespace(infer=infer, mm=mm, cfg=cfg)
+def gold():
+    g = np.load(GOLD)
+    t = {k: torch.from_numpy(g[k]).to(torch.bfloat16) for k in g.files if k != "meta"}     # bf16 values stored as f32
+    return t, json.loads(str(g["meta"]))
 
 
 @pytest.fixture()
 def engines(pkg, monkeypatch):
     """B200NaDiT / B200VideoVAE built on the CPU with the kernel layer replaced by the oracle (test double)."""
+    return dropin.slot_engines(pkg, monkeypatch)
+
+
+def test_reference_runner_drives_the_engine_slots(pkg, engines, gold):
+    """One clip through the reference's own VideoDiffusionInfer with the engine modules in its slots (as recorded), and
+    the same clip through the engine's own runner."""
     from oracle import dit_oracle, vae_oracle
-    lib = importlib.import_module("comfyui_seedvr2_videoupscaler_b200.lib")
-    dit = importlib.import_module("comfyui_seedvr2_videoupscaler_b200.dit")
-    vae = importlib.import_module("comfyui_seedvr2_videoupscaler_b200.vae")
-    monkeypatch.setattr(lib, "device_check", lambda: (148, 10, 0))
-
-    def fake_linear(a, w, *, bias=None, epi=0, **kw):          # the three load-time time-embedding GEMMs
-        y = a.float() @ w.float().T + (bias.float() if bias is not None else 0)
-        y = y.to(torch.bfloat16)
-        return torch.nn.functional.silu(y.float()).to(torch.bfloat16) if epi & lib.EPI_SILU else y
-    monkeypatch.setattr(lib, "linear", fake_linear)
-    over = dict(dim=256, heads=2, layers=4, mm_layers=2, txt_in_dim=64)
-    cfg = dit.dit_config("3b", **over)
-    dsd = pkg.weights.synth_dit_state_dict(cfg, seed=1234, dtype=torch.float16)
-    vsd = pkg.weights.synth_vae_state_dict(seed=4321, dtype=torch.float16)
-    d, v = dit.B200NaDiT(cfg, dsd, device="cpu"), vae.B200VideoVAE(vsd, device="cpu")
-    calls = {"dit": [], "enc": [], "dec": []}
-    ocfg = dit_oracle.dit_config("3b", **over)
-    d32, v32 = {k: t.float() for k, t in dsd.items()}, {k: t.float() for k, t in vsd.items()}
-
-    def dit_forward(self, vid, txt, vid_shape, txt_shape, timestep=None, disable_cache=False):
-        calls["dit"].append(dict(vid=tuple(vid.shape), txt=tuple(txt.shape), vid_shape=vid_shape.tolist(),
-                                 txt_shape=txt_shape.tolist(), timestep=timestep.tolist(), dtype=vid.dtype))
-        (T, H, W), = vid_shape.tolist()
-        return dit.NaDiTOutput(dit_oracle.dit_forward(d32, ocfg, vid.float(), txt.float(), T, H, W).to(vid.dtype))
-
-    def enc(self, x, return_dict=True, tiled=False, tile_size=None, tile_overlap=None):
-        calls["enc"].append(dict(shape=tuple(x.shape), tiled=tiled, tile_size=tile_size, tile_overlap=tile_overlap))
-        return vae.VAEOutput(latent=vae_oracle.vae_encode(v32, x.float()).to(x.dtype).squeeze(2), latent_dist=None)
-
-    def dec(self, z, return_dict=True, tiled=False, tile_size=None, tile_overlap=None):
-        calls["dec"].append(dict(shape=tuple(z.shape), tiled=tiled, tile_size=tile_size, tile_overlap=tile_overlap))
-        z5 = z.unsqueeze(2) if z.ndim == 4 else z
-        return vae.VAEOutput(sample=vae_oracle.vae_decode(v32, z5.float()).to(z.dtype).squeeze(2))
-    monkeypatch.setattr(dit.B200NaDiT, "forward", dit_forward)
-    monkeypatch.setattr(vae.B200VideoVAE, "encode", enc)
-    monkeypatch.setattr(vae.B200VideoVAE, "decode", dec)
-    return types.SimpleNamespace(dit=d, vae=v, calls=calls, d32=d32, v32=v32, ocfg=ocfg)
+    t, meta = gold
+    assert meta["runner"] == dict(encode_tiled=False, decode_tiled=True, decode_tile_size=[64, 64],
+                                  decode_tile_overlap=[16, 16])
+    # the calls the reference runner made, bound against the engine's real methods
+    enc, dit_call, dec = meta["contract"]
+    assert [c["slot"] for c in meta["contract"]] == ["enc", "dit", "dec"]
+    modules = {"enc": engines.vae, "dit": engines.dit, "dec": engines.vae}
+    for c in meta["contract"]:
+        inspect.signature(engines.real[c["slot"]]).bind(modules[c["slot"]], *[None] * c["positional"],
+                                                        **{k: None for k in c["keywords"]})
+    assert enc["args"]["x"]["tensor"] == [1, 3, 5, 32, 48] and enc["args"]["tiled"] is False
+    a = dit_call["args"]
+    assert a["vid"]["tensor"] == [2 * 4 * 6, 33] and a["txt"]["tensor"] == [58, 64] and a["vid"]["dtype"] == "bfloat16"
+    assert a["vid_shape"]["values"] == [2, 4, 6] and a["txt_shape"]["values"] == [58]
+    assert a["timestep"]["values"] == [1000.0]                                              # the t the engine folds at load
+    assert dec["args"]["z"]["tensor"] == [1, 16, 2, 4, 6]
+    assert (dec["args"]["tiled"], dec["args"]["tile_size"], dec["args"]["tile_overlap"]) == (True, [64, 64], [16, 16])
+    # what the reference runner returned, against the oracle
+    assert tuple(t["lat"].shape) == (2, 4, 6, 16)                                           # t h w c, scaled by 0.9152
+    assert (t["lat"].float() - vae_oracle.runner_encode(engines.v32, t["clip"][None].float())).abs().max() < 0.05
+    vid = torch.cat([t["noise"], t["cond"]], -1).reshape(-1, 33).float()
+    v = dit_oracle.dit_forward(engines.d32, engines.ocfg, vid, t["txt"].float(), 2, 4, 6)
+    assert (t["x0"].float() - dit_oracle.one_step_latent(t["noise"].float(), v.view(2, 4, 6, 16))).abs().max() < 0.1
+    assert tuple(t["sample"].shape) == (3, 5, 32, 48)
+    # the engine's own runner on the same clip, noise and text reproduces the reference runner's phases: up to two bf16
+    # ulps, since the oracle's fp32 sums on another CPU (other vector width, other thread count) round a few values the
+    # other way
+    pipeline = importlib.import_module("comfyui_seedvr2_videoupscaler_b200.pipeline")
+    eng = object.__new__(pipeline.SeedVR2Engine)
+    eng.device, eng.dit, eng.vae, eng.txt = torch.device("cpu"), engines.dit, engines.vae, t["txt"]
+    for got, want in ((eng.vae_encode(t["clip"]), t["lat"]), (eng.inference(t["noise"], t["lat"]), t["x0"]),
+                      (eng.vae_decode(t["x0"]), t["sample"])):
+        assert got.dtype == torch.bfloat16
+        torch.testing.assert_close(got.float(), want.float(), rtol=2 ** -6, atol=2 ** -8)
+    assert [c["slot"] for c in engines.contract] == ["enc", "dit", "dec"]
 
 
-def test_reference_runner_drives_the_engine_slots(ref, engines):
-    """One clip through the reference's own VideoDiffusionInfer with the engine modules in its slots."""
-    from oracle import dit_oracle, vae_oracle
-    runner = ref.infer.VideoDiffusionInfer(ref.cfg, Debug(), encode_tiled=False, decode_tiled=True,
-                                           decode_tile_size=(64, 64), decode_tile_overlap=(16, 16))
-    runner.dit, runner.vae = engines.dit, engines.vae
-    runner.configure_diffusion(device=torch.device("cpu"), dtype=torch.bfloat16)
-    g = torch.Generator().manual_seed(3)
-    clip = (torch.rand(3, 5, 32, 48, generator=g) * 2 - 1).to(torch.bfloat16)            # c t h w (generation_phases.py:489)
-    lat, = runner.vae_encode([clip])
-    assert tuple(lat.shape) == (2, 4, 6, 16) and lat.dtype == torch.bfloat16              # t h w c, scaled by 0.9152
-    want = vae_oracle.runner_encode(engines.v32, clip[None].float())
-    assert (lat.float() - want).abs().max() < 0.05
-    noise = torch.randn(lat.shape, generator=g).to(torch.bfloat16)
-    cond = runner.get_condition(noise, task="sr", latent_blur=lat)
-    txt = torch.randn(58, 64, generator=g).to(torch.bfloat16)
-    x0, = runner.inference(noises=[noise], conditions=[cond], texts_pos=[txt], texts_neg=[txt])
-    call, = engines.calls["dit"]
-    assert call["vid"] == (2 * 4 * 6, 33) and call["txt"] == (58, 64) and call["vid_shape"] == [[2, 4, 6]]
-    assert call["txt_shape"] == [[58]] and call["timestep"] == [1000.0]                    # the t the engine folds at load
-    vid = torch.cat([noise, cond], -1).reshape(-1, 33).float()
-    v = dit_oracle.dit_forward(engines.d32, engines.ocfg, vid, txt.float(), 2, 4, 6)
-    assert (x0.float() - dit_oracle.one_step_latent(noise.float(), v.view(2, 4, 6, 16))).abs().max() < 0.1
-    out, = runner.vae_decode([x0])
-    assert tuple(out.shape) == (3, 5, 32, 48)
-    assert engines.calls["enc"][0]["tiled"] is False
-    assert engines.calls["dec"][0] == dict(shape=(1, 16, 2, 4, 6), tiled=True, tile_size=(64, 64), tile_overlap=(16, 16))
-
-
-def test_module_surface_and_lifecycle(ref, engines):
-    mm = ref.mm
+def test_module_surface_and_lifecycle(engines, gold):
+    _, meta = gold
     d, v = engines.dit, engines.vae
     for m in (d, v):
         assert isinstance(m, torch.nn.Module)
@@ -165,16 +95,25 @@ def test_module_surface_and_lifecycle(ref, engines):
     hits = [mod for mod in d.modules() if type(mod).__name__ == "FlashAttentionVarlen"]
     assert len(hits) == 1
     hits[0].attention_mode, hits[0].compute_dtype = "sdpa", torch.bfloat16
-    assert mm.clear_rope_lru_caches(d) == 0                       # walks named_modules() without tripping
-    n_buf = sum(b.numel() for b in d.buffers())
-    mm.manage_model_device(model=d, target_device=torch.device("cpu"), model_name="DiT", debug=Debug(), reason="test")
-    assert sum(b.numel() for b in d.buffers()) == n_buf
+    # clear_rope_lru_caches counts the modules with a cached get_axial_freqs; it found none
+    life = meta["lifecycle"]
+    assert life["clear_rope_lru_caches"]["returned"] == 0
+    assert not [n for n, mod in d.named_modules() if hasattr(getattr(mod, "get_axial_freqs", None), "cache_clear")]
+    # manage_model_device moved nothing: the parameters already sit on the target device
+    assert life["manage_model_device"]["returned"] is False and next(d.parameters()).device == torch.device("cpu")
+    # every module call the lifecycle functions made, replayed on the engine modules: none fails, nothing is dropped
+    n_buf = {id(m): sum(b.numel() for b in m.buffers()) for m in (d, v)}
+    for tag in ("clear_rope_lru_caches", "manage_model_device", "cleanup_dit", "cleanup_vae"):
+        for key, m in (("dit", d), ("vae", v)):
+            for call in life[tag].get(key, []):
+                r = getattr(m, call["method"])(*dropin.unplain(call["args"]),
+                                               **{k: dropin.unplain(x) for k, x in call["kwargs"].items()})
+                if inspect.isgenerator(r):
+                    list(r)
+    assert {c["method"] for c in life["cleanup_dit"]["dit"]} >= {"named_modules", "parameters", "zero_grad", "buffers"}
+    for m in (d, v):
+        assert sum(b.numel() for b in m.buffers()) == n_buf[id(m)]
     # offloaded / released weights must fail loudly, never fall back
     lib = importlib.import_module("comfyui_seedvr2_videoupscaler_b200.lib")
     with pytest.raises(lib.Svr2Error):
         d._require_cuda("forward")
-    runner = types.SimpleNamespace(dit=d, vae=v, sampler=1, schedule=1, sampling_timesteps=1)
-    mm.cleanup_dit(runner, debug=Debug(), cache_model=False)      # memory_manager.py:1011-1097
-    assert runner.dit is None and runner.sampler is None
-    mm.cleanup_vae(runner, debug=Debug(), cache_model=False)
-    assert runner.vae is None
