@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libsvr2.so")
-SOURCES = ["api.cu", "gemm.cu", "attn.cu", "elementwise.cu", "post.cu", "pre.cu", "engine.cu", "vae_engine.cu"]
+SOURCES = ["api.cu", "gemm.cu", "attn.cu", "elementwise.cu", "post.cu", "pre.cu", "alpha.cu", "engine.cu", "vae_engine.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

@@ -17,7 +17,7 @@
 namespace svr2 {
 namespace {
 
-constexpr int kMaxTaps = 32;
+constexpr int kMaxTaps = kAaMaxTaps;
 
 __device__ __forceinline__ float rn(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
@@ -127,20 +127,26 @@ __global__ void __launch_bounds__(256) resize_kernel(const T* __restrict__ in, _
 }
 
 inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
-inline int taps_for(int in_size, int out_size) {
+
+}  // namespace
+
+int aa_taps(int in_size, int out_size) {
   const float scale = (float)in_size / (float)out_size;
   const float support = scale >= 1.0f ? 2.0f * scale : 2.0f;
   return (int)ceilf(support) * 2 + 1;
 }
 
-}  // namespace
+void aa_tables(int in_size, int out_size, int K, int* first, int* count, float* weights, cudaStream_t s) {
+  aa_table_kernel<<<(out_size + 127) / 128, 128, 0, s>>>(in_size, out_size, K, first, count, weights);
+}
+
 }  // namespace svr2
 
 using namespace svr2;
 
 extern "C" int64_t svr2_resize_scratch_bytes(int h, int w, int H, int W) {
   if (h <= 0 || w <= 0 || H <= 0 || W <= 0) return 0;
-  const int K = taps_for(h, H) > taps_for(w, W) ? taps_for(h, H) : taps_for(w, W);
+  const int K = aa_taps(h, H) > aa_taps(w, W) ? aa_taps(h, H) : aa_taps(w, W);
   return (int64_t)(2 * align256((size_t)(H > W ? H : W) * 2 * sizeof(int)) +
                    2 * align256((size_t)(H > W ? H : W) * K * sizeof(float)));
 }
@@ -151,7 +157,7 @@ extern "C" int svr2_resize_bicubic_aa_bf16(const void* in, int in_dtype, int cha
   if (frames <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0) return set_error(SVR2_ERR_ARG, "svr2_resize: empty image");
   if (frames > 65535) return set_error(SVR2_ERR_ARG, "svr2_resize: at most 65535 frames per call");
   if (cin < 3 || (!channels_last && cin != 3)) return set_error(SVR2_ERR_ARG, "svr2_resize: need >= 3 channels");
-  const int K = taps_for(h, H) > taps_for(w, W) ? taps_for(h, H) : taps_for(w, W);
+  const int K = aa_taps(h, H) > aa_taps(w, W) ? aa_taps(h, H) : aa_taps(w, W);
   if (K > kMaxTaps) return set_error(SVR2_ERR_ARG, "svr2_resize: down-scale factor too large (> 7x)");
   if (!scratch || scratch_bytes < svr2_resize_scratch_bytes(h, w, H, W))
     return set_error(SVR2_ERR_ARG, "svr2_resize: scratch too small (svr2_resize_scratch_bytes)");
@@ -165,8 +171,8 @@ extern "C" int svr2_resize_bicubic_aa_bf16(const void* in, int in_dtype, int cha
   int* ycount = yfirst + L;
   float* xw = (float*)(base + 2 * seg_i);
   float* yw = (float*)(base + 2 * seg_i + seg_w);
-  aa_table_kernel<<<(W + 127) / 128, 128, 0, s>>>(w, W, K, xfirst, xcount, xw);
-  aa_table_kernel<<<(H + 127) / 128, 128, 0, s>>>(h, H, K, yfirst, ycount, yw);
+  aa_tables(w, W, K, xfirst, xcount, xw, s);
+  aa_tables(h, H, K, yfirst, ycount, yw, s);
   int rc = check_launch("aa_table");
   if (rc) return rc;
   const int Hp = finish ? (H + 15) / 16 * 16 : H, Wp = finish ? (W + 15) / 16 * 16 : W;

@@ -20,6 +20,11 @@ int ndhwc_to_ncdhw_strided(const void* in, int ld_in, int C, int T, int H, int W
                            int64_t chan_stride, void* stream);
 int conv_tap_gather_strided(const float* z, int64_t ldz, int co_n, const void* bias, int T, int H, int W, void* out,
                             int out_dtype, int64_t chan_stride, void* stream);
+// pre.cu: tap tables of torch's antialiased bicubic resize (_upsample_bicubic2d_aa) along one axis, laid out as
+// first[out], count[out], weights[out][K]; K = the larger aa_taps() of the two axes, at most kAaMaxTaps
+constexpr int kAaMaxTaps = 32;
+int aa_taps(int in_size, int out_size);
+void aa_tables(int in_size, int out_size, int K, int* first, int* count, float* weights, cudaStream_t s);
 inline int check_launch(const char* what) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {

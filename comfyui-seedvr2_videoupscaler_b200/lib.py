@@ -96,6 +96,11 @@ SIGNATURES = {
     "svr2_resize_scratch_bytes": [c_int, c_int, c_int, c_int],
     "svr2_resize_bicubic_aa_bf16": [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, c_int, _P, c_int64,
                                     _P],
+    "svr2_alpha_scratch_bytes": [c_int, c_int, c_int, c_int, c_int],
+    "svr2_alpha_resize_f32": [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, _P, c_int64, _P],
+    "svr2_alpha_edges_u8": [_P, c_int, c_int64, c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int64, _P],
+    "svr2_alpha_refine": [_P, c_int, c_int64, c_int64, c_int64, _P, _P, c_int, c_int, c_int, c_int, c_int, _P, c_int,
+                          c_int, _P, c_int64, _P],
 }
 
 _lib = None
@@ -141,7 +146,10 @@ def stream():
 KERNELS_PER_CALL = {"svr2_groupnorm_bf16": 3, "svr2_groupnorm_from_stats_bf16": 2,
                     "svr2_resize_bicubic_aa_bf16": 3,      # two tap-table kernels + the resize
                     "svr2_adain_bf16": 2,                  # statistics + apply
-                    "svr2_histogram_match_f32": 2}         # iota + rank scatter (the CUB radix-sort passes are library launches)
+                    "svr2_histogram_match_f32": 2,         # iota + rank scatter (the CUB radix-sort passes are library launches)
+                    "svr2_alpha_resize_f32": 4,            # two tap-table kernels + the binary-mask count + the resize
+                    "svr2_alpha_edges_u8": 2,              # flags / per-frame maxima + the edge map
+                    "svr2_alpha_refine": 2}                # the two guided-filter box passes
 
 
 class Profiler:

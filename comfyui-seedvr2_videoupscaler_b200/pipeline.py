@@ -7,7 +7,8 @@ between phases on the device (no host bounce).  ``upscale_clip`` strings them
 together the way ``generation_phases.py`` does for one clip: 4n+1 temporal pad
 (:109-124), clamp + pad-16 + normalise (``generation_utils.py:72-84``), encode,
 condition = [latent | 1] (``infer.py:54-78``), DiT, decode, crop, optional colour
-correction against the input clip (``generation_phases.py:1249-1319``), [0,1] image format.
+correction against the input clip (``generation_phases.py:1249-1319``), [0,1] image format, and with ``keep_alpha`` the
+edge-guided upscale of an RGBA clip's alpha (``generation_phases.py:1142-1217``).
 """
 from __future__ import annotations
 
@@ -15,6 +16,7 @@ from typing import Dict, Optional
 
 import torch
 
+from . import alpha as alpha_ops
 from . import color_fix, preprocess
 from .dit import B200NaDiT, dit_config
 from .vae import B200VideoVAE
@@ -114,16 +116,34 @@ class SeedVR2Engine:
     @torch.no_grad()
     def upscale_clip(self, frames: torch.Tensor, noise: Optional[torch.Tensor] = None, seed: int = 42,
                      color_correction: str = "none", resolution: Optional[int] = None,
-                     max_resolution: int = 0) -> torch.Tensor:
-        """frames (T,h,w,3) in [0,1]; ``resolution`` = target shortest edge (None: keep the size, i.e. the frames
+                     max_resolution: int = 0, keep_alpha: bool = False) -> torch.Tensor:
+        """frames (T,h,w,C>=3) in [0,1]; ``resolution`` = target shortest edge (None: keep the size, i.e. the frames
         are already at the target resolution).  Returns (T,H,W,3) bf16 in [0,1] on the device.
         ``color_correction``: "none", "lab" (the reference CLI default), "wavelet" or "adain" — matched against the
-        transformed input clip (generation_phases.py:1299-1317)."""
+        transformed input clip (generation_phases.py:1299-1317).
+        ``keep_alpha`` with 4-channel frames: returns (T,H,W,4), the RGB of the 3-channel result plus channel 3 upscaled
+        by ``alpha.upscale_alpha`` against the decoded sample before colour correction."""
         sample, style = self.clip_to_sample(frames, noise=noise, seed=seed, resolution=resolution,
                                             max_resolution=max_resolution)
+        return self._finish(sample, style, color_correction, frames if keep_alpha else None)
+
+    def _finish(self, sample: torch.Tensor, style: torch.Tensor, color_correction: str,
+                frames: Optional[torch.Tensor]) -> torch.Tensor:
+        """Phase 4 of one slice: with RGBA ``frames`` (the source frames of exactly this slice) the alpha is upscaled
+        against the sample first, then colour correction and the [0,1] image format."""
+        rgba = None
+        if frames is not None and frames.shape[-1] == 4:
+            src = frames if frames.is_cuda else frames[..., 3:].to(self.device)
+            T, _, H, W = sample.shape
+            rgba = torch.empty(T, H, W, 4, device=sample.device, dtype=torch.bfloat16)
+            alpha_ops.upscale_alpha(src, src.shape[-1] - 1, sample, out=rgba[..., 3])
         if color_correction != "none":
             sample = color_fix.apply_color_correction(sample, style, color_correction)
-        return color_fix.sample_to_image(sample)                    # t h w c in [0,1]
+        rgb = color_fix.sample_to_image(sample)                     # t h w c in [0,1]
+        if rgba is None:
+            return rgb
+        rgba[..., :3] = rgb
+        return rgba
 
     @torch.no_grad()
     def clip_to_sample(self, frames: torch.Tensor, noise: Optional[torch.Tensor] = None, seed: int = 42,
@@ -155,21 +175,26 @@ class SeedVR2Engine:
     @torch.no_grad()
     def upscale_video(self, frames: torch.Tensor, batch_size: int = 5, temporal_overlap: int = 0, seed: int = 42,
                       color_correction: str = "none", resolution: Optional[int] = None,
-                      max_resolution: int = 0) -> torch.Tensor:
+                      max_resolution: int = 0, keep_alpha: bool = False) -> torch.Tensor:
         """A whole video on one GPU the way the reference's four phases do it (generation_phases.py:271-289, 344-358,
         969-1000, 1236-1345): batches of ``batch_size`` frames stepping by ``batch_size - temporal_overlap``, every batch
         seeded identically, the overlap cross-faded into the previous batch's tail, colour correction per batch
-        against its own input frames, [0,1] image format.  Returns (T,H,W,3) bf16."""
+        against its own input frames, [0,1] image format.  Returns (T,H,W,3) bf16, or (T,H,W,4) with ``keep_alpha``
+        and 4-channel frames: each written slice's alpha comes from the source frames of that slice (the reference
+        passes the whole batch's alpha and fails to broadcast when overlap frames were dropped or the batch was
+        padded to 4n+1)."""
         from . import shard
 
         def clip(a, b):
             s, st = self.clip_to_sample(frames[a:b], seed=seed, resolution=resolution, max_resolution=max_resolution)
             return s.contiguous(), st.contiguous()
 
+        written = [0]                           # run_batched post-processes the slices in order, laid end to end
+
         def post(sample, style):
-            if color_correction != "none":
-                sample = color_fix.apply_color_correction(sample, style, color_correction)
-            return color_fix.sample_to_image(sample)
+            a = written[0]
+            written[0] += sample.shape[0]
+            return self._finish(sample, style, color_correction, frames[a:written[0]] if keep_alpha else None)
 
         return run_batched(frames.shape[0], batch_size, temporal_overlap, clip, shard.blend_overlap, post)
 

@@ -324,6 +324,30 @@ int64_t svr2_resize_scratch_bytes(int h, int w, int H, int W);
 int svr2_resize_bicubic_aa_bf16(const void* in, int in_dtype, int channels_last, int cin, int frames, int h, int w,
                                 void* out, int H, int W, int finish, void* scratch, int64_t scratch_bytes, void* stream);
 
+/* ---- Alpha of RGBA clips (edge_guided_alpha_upscale, src/core/alpha_upscaling.py:289-438).
+ * Three stages over one caller-owned scratch of svr2_alpha_scratch_bytes(T, h, w, H, W) bytes: the stages leave the
+ * batch-wide decisions (binary mask; [-1,1] -> [0,1] normalisation of the RGB, once or twice) there as device flags,
+ * so svr2_alpha_refine must run after svr2_alpha_resize_f32 and svr2_alpha_edges_u8 on the same scratch and stream.
+ * No stage synchronises with the host.  The RGB is the decoded sample [T,3,H,W] before colour correction, fp32 or
+ * bf16 (rgb_dtype 0 | 1) with element strides between channels, frames and rows (pixels contiguous).
+ *   svr2_alpha_resize_f32: source alpha = channel `channel` of [T,h,w,channels] (channels > 0) or [T,1,h,w]
+ *     (channels == 0), dtype 0 fp32 | 1 bf16 | 2 fp16, rounded to bf16 on load -> out [T,H,W] fp32 = antialiased
+ *     bicubic (torch _upsample_bicubic2d_aa) then clamp(0,1); also counts the source alpha < 0.1 and > 0.9.
+ *   svr2_alpha_edges_u8: edges [T,H,W] u8 = the reference's Sobel edge map (cv2 RGB2GRAY, Sobel 3x3 with
+ *     BORDER_REFLECT_101, magnitude / per-frame maximum * 255 truncated, 0 for a frame without edges), bit-exact.
+ *   svr2_alpha_refine: guided filter of the resized alpha by the mean of the normalised RGB (eps 0.002, radius 2 for
+ *     a binary mask, else 3), the binary-mask refinement, clamp(0,1) -> out element ((t*H + y)*W + x) * out_stride,
+ *     out_dtype 0 fp32 | 1 bf16 (out_stride 1: [T,1,H,W]; 4 with out at channel 3: the alpha of [T,H,W,4]). */
+int64_t svr2_alpha_scratch_bytes(int frames, int h, int w, int H, int W);
+int svr2_alpha_resize_f32(const void* alpha, int dtype, int channels, int channel, int frames, int h, int w, float* out,
+                          int H, int W, void* scratch, int64_t scratch_bytes, void* stream);
+int svr2_alpha_edges_u8(const void* rgb, int rgb_dtype, int64_t chan_stride, int64_t frame_stride, int64_t row_stride,
+                        int frames, int h, int w, int H, int W, uint8_t* edges, void* scratch, int64_t scratch_bytes,
+                        void* stream);
+int svr2_alpha_refine(const void* rgb, int rgb_dtype, int64_t chan_stride, int64_t frame_stride, int64_t row_stride,
+                      const float* alpha_up, const uint8_t* edges, int frames, int h, int w, int H, int W, void* out,
+                      int out_dtype, int out_stride, void* scratch, int64_t scratch_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
